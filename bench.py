@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W          (N>1 under torchrun)
   python bench.py --impl reference ...                   (CPU oracle arm)
+  python bench.py ... --dump-outputs DIR                 (outputs of the last timed step as .npy)
 
 A "step" is one cold solve of the whole batch (BASELINE config 2: batch 1024
 Holonomic Point2point, 10 knot intervals, 3 circular obstacles) from the linear
@@ -24,6 +25,7 @@ sys.path.insert(0, ROOT)
 
 BATCH = 1024
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 64 << 20
 
 
 def parse():
@@ -44,6 +46,10 @@ def parse():
     ap.add_argument('--formations', type=int, default=1,
                     help='config3: independent formations run side by side in one batch (value counts '
                          'formation-iterations; 9 x 64 agents fill the 592 resident blocks of one B200)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step computed (rank 0) as '
+                         'DIR/<name>.npy in float64, at most 64 MiB in all, so that two builds can be '
+                         'compared output for output on the same inputs')
     args = ap.parse_args()
     if args.batch <= 0:
         args.batch = {'config4': 512, 'config4_5obs': 512, 'config5': 256}.get(args.workload, BATCH)
@@ -100,6 +106,25 @@ class ClockSampler(object):
         return {'sm_mhz': float(np.median(sm)) if sm else None,
                 'sm_max_mhz': max(mx) if mx else None, 'reasons': reasons,
                 'samples': len(self.rows)}
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy in float64 (status and iteration counts are
+    exact there).  Above DUMP_BYTES in all, the per-instance arrays (leading axis = the batch)
+    keep the same rows, a sample drawn with a fixed seed, so that two runs keep the same rows."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    B = max(len(a) for a in arrays.values() if a.ndim > 0)
+    per_instance = [k for k, a in arrays.items() if a.ndim > 0 and len(a) == B]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        row_bytes = sum(arrays[k].nbytes for k in per_instance) // B
+        keep = max(1, (DUMP_BYTES - (total - B * row_bytes)) // row_bytes)
+        rows = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        for k in per_instance:
+            arrays[k] = arrays[k][rows]
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def roofline_bytes_per_solve(tb, K):
@@ -259,6 +284,10 @@ def run_config3(args, rank, world, dev):
         dist.all_reduce(tm, op=dist.ReduceOp.MAX)
     st, it = run.status()
     per = run.formation_residuals()          # collective: every rank
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'residuals': res, 'x': run.X.cpu(), 'z_i': run.z_i.cpu(),
+                                         'z_ij': run.z_ij.cpu(), 'l_i': run.l_i.cpu(),
+                                         'l_ij': run.l_ij.cpu(), 'status': st, 'iters': it})
     if rank == 0:
         ms = float(tm[0])
         tb = pr.tb
@@ -311,6 +340,8 @@ def run_reference(args, rank, world):
         dt = time.perf_counter() - t0
         if k >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'x': info['x'], 'status': info['status'], 'iters': info['iters']})
     tot = sum(times)
     value = sample * args.steps / tot
     line = {
@@ -407,6 +438,9 @@ def main():
     kern_ms = tot_ms / args.steps       # one kernel launch per step
     iters = IT.cpu().numpy()
     status = ST.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'x': X.cpu(), 'lam_g': LAM.cpu(), 'f': F.cpu(),
+                                         'status': status, 'iters': iters})
     # ---- e2e: host buffers through the C-ABI call --------------------------------
     pin = lambda a: torch.from_numpy(a).pin_memory().numpy()
     X0p, Pp = pin(X0h), pin(Ph)

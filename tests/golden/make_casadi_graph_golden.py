@@ -223,8 +223,14 @@ def record(name):
         emit(r)
         ops.append(OPS['OP_OUTPUT']); ins.append((r.w, 0)); outs.append((1, i)); consts.append(0.0)
     print(name, 'n', n, 'n_par', n_par, 'm', len(rows), 'nodes created', Node.count, 'instructions', len(ops))
-    return {'ops': np.array(ops, np.int16), 'ins': np.array(ins, np.int32), 'outs': np.array(outs, np.int32),
-            'consts': np.array(consts), 'sizes': np.array([n, n_par, len(rows), counter[0]]),
+    # stored compactly to keep the file small: the constant of the OP_CONST rows and the output
+    # slot of the OP_OUTPUT rows only (every other row writes its own work index and has no
+    # constant); tests/test_lower_casadi.py restores the full lists
+    ops = np.array(ops, np.int16)
+    return {'ops': ops, 'ins': np.array(ins, np.int32),
+            'output_slots': np.array(outs, np.int32)[ops == OPS['OP_OUTPUT']],
+            'const_values': np.array(consts)[ops == OPS['OP_CONST']],
+            'sizes': np.array([n, n_par, len(rows), counter[0]]),
             'lb': np.array(lb), 'ub': np.array(ub)}
 
 

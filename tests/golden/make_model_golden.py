@@ -679,7 +679,7 @@ def shape_zoo(shp):
 
 BASE_NAMES = ('config1', 'config2', 'config4', 'config5', 'config_holonomic3d',
               'config_quadrotor2d', 'config_dubins')
-# second fixture file (model_golden_ext.npz, `--ext`): formulations whose rows multiply the
+# second set of fixture files (model_golden_ext1..3.npz, `--ext`): formulations whose rows multiply the
 # intermediates by decision variables
 EXT_NAMES = ('config_dubins_plain', 'config_dubins_rect', 'config_dubins_exact',
              'config_holonomic_orient', 'config_bicycle', 'config_agv',
@@ -692,7 +692,7 @@ EXT_NAMES = ('config_dubins_plain', 'config_dubins_rect', 'config_dubins_exact',
 def main(ext=False):
     global REG
     install_stubs()
-    out = {}
+    out, owner = {}, {}
     n_samples = 3
     for name in (EXT_NAMES if ext else BASE_NAMES):
         Xs, Ps, Gs, Fs = [], [], [], []
@@ -741,10 +741,13 @@ def main(ext=False):
         out[name + '_lb'], out[name + '_ub'] = lb, ub
         out[name + '_var_layout'] = np.array(['%s|%s|%dx%d' % ((lab, nm) + v.a.shape) for lab, nm, v in var])
         out[name + '_par_layout'] = np.array(['%s|%s|%dx%d' % ((lab, nm) + v.a.shape) for lab, nm, v in par])
+        owner.update((k, name) for k in out if k not in owner)
     if ext:
-        path = OUT.replace('model_golden.npz', 'model_golden_ext.npz')
-        np.savez_compressed(path, **out)
-        print('wrote', path)
+        # three files of whole models, each below 1 MB
+        for part, names in enumerate((EXT_NAMES[:7], EXT_NAMES[7:15], EXT_NAMES[15:])):
+            path = OUT.replace('model_golden.npz', 'model_golden_ext%d.npz' % (part + 1))
+            np.savez_compressed(path, **{k: v for k, v in out.items() if owner[k] in names})
+            print('wrote', path, os.path.getsize(path), 'bytes')
         return
     # Fleet of the formation examples (vehicles/fleet.py: set_configuration, neighbours)
     hol, fl = ref_import('vehicles.holonomic'), ref_import('vehicles.fleet')

@@ -25,7 +25,15 @@ class RecordedSXFunction(object):
 
     def __init__(self, G, name):
         self.ops, self.ins = G[name + '_ops'], G[name + '_ins']
-        self.outs, self.consts = G[name + '_outs'], G[name + '_consts']
+        # the file keeps the constants of OP_CONST and the slots of OP_OUTPUT only; every other
+        # instruction writes the next entry of the work vector and has the constant 0
+        code = {str(nm): int(c) for nm, c in zip(G['op_names'], G['op_codes'])}
+        is_const, is_out = self.ops == code['OP_CONST'], self.ops == code['OP_OUTPUT']
+        self.consts = np.zeros(len(self.ops))
+        self.consts[is_const] = G[name + '_const_values']
+        self.outs = np.zeros((len(self.ops), 2), np.int32)
+        self.outs[~is_out, 0] = np.arange(np.count_nonzero(~is_out))
+        self.outs[is_out] = G[name + '_output_slots']
         self.n, self.n_par, self.m, self.w = [int(v) for v in G[name + '_sizes']]
 
     def n_instructions(self): return len(self.ops)

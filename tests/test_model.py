@@ -869,9 +869,16 @@ def _cached_problem(name):
 
 
 def _model_golden(name):
+    """The fixture file holding `name` (make_model_golden.py --ext splits the ext models over three
+    files, each below 1 MB)."""
     import os
-    fn = 'model_golden_ext.npz' if name in EXT_GOLDEN else 'model_golden.npz'
-    return np.load(os.path.join(os.path.dirname(__file__), 'golden', fn))
+    files = ('model_golden_ext1.npz', 'model_golden_ext2.npz', 'model_golden_ext3.npz') \
+        if name in EXT_GOLDEN else ('model_golden.npz',)
+    for fn in files:
+        M = np.load(os.path.join(os.path.dirname(__file__), 'golden', fn))
+        if name + '_var_layout' in M.files:
+            return M
+    raise KeyError(name)
 
 
 @pytest.mark.parametrize('name', ['config1', 'config2', 'config4', 'config5', 'config_holonomic3d',
