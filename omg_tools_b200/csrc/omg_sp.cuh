@@ -931,6 +931,10 @@ __device__ __forceinline__ void ipm_body_sp(const DevTab& T, const SpTab& P, con
         sp_factor(T, P, S, &ctl, fflags, O.inertia_mode, tracing ? phase_cyc : nullptr);
         TICK(7);
         if (!ctl.fail) break;
+        // the failed attempt wrote LK through the generic proxy; the next staging overwrites it
+        // through the async proxy (cp.async.bulk): every writer orders its writes before the
+        // barrier that precedes the copy (PTX memory model, proxy fence)
+        sp_fence_async();
         if (tid == 0) {
           if (ctl.eq_fail) ctl.delta_c = DELTA_C_VAL * pow(mu, DELTA_C_EXP);
           if (ctl.first_try) {

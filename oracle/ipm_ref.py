@@ -164,7 +164,9 @@ def solve(tb, x0, p, lbg=None, ubg=None, options=None, lam_g0=None,
                    np.max(np.where(hasL | is_eq, lbg - g_un, 0.0))) if m else 0.0
         dinf_un = max(np.abs(r_x).max(), (np.abs(r_s) * dsc).max() if m else 0.0) / fsc
         if trace:
-            log.append((it, f / fsc, cinf, dinf, mu, E0))
+            # (iter, f, cinf, dinf, mu, E0, alpha, delta_w): the last two belong to the step
+            # taken FROM this iterate and are filled in below (0.0 while there is none)
+            log.append((it, f / fsc, cinf, dinf, mu, E0, 0.0, 0.0))
         if not np.isfinite(E0):
             status = 4
             break
@@ -331,6 +333,8 @@ def solve(tb, x0, p, lbg=None, ubg=None, options=None, lam_g0=None,
                     filt = []
                     break
                 alpha *= 0.5
+        if trace:
+            log[-1] = log[-1][:6] + (alpha if accepted else 0.0, delta_w)
         if not accepted:
             if n_restarts < o['max_restarts']:
                 # feasibility restart (stand-in for IPOPT's restoration phase): keep x,
